@@ -2,6 +2,7 @@
 """bench.py — benchmark of the GP-posterior + acquisition hot path (contract: see the prompt / DESIGN.md §6).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--config headline|c2|c3|c4|c5] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 headline (default, the driver's run)
   metric  : acquisition candidate-points/sec, ExpectedImprovement on an exact GPR with N=4096 training points, fp64
@@ -37,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 N_TRAIN = 4096
 DIM = 10
@@ -283,6 +285,24 @@ def load_peaks():
         return {}
 
 
+# 16 MB of float64 values + 16 MB of row numbers; a dump holds at most one array this long, so it stays below 64 MB
+DUMP_MAX_ROWS = 2_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array of ``arrays`` (name -> array or scalar) as ``out_dir/<name>.npy`` in float64; indices are exact
+    below 2**53.  An array of more than DUMP_MAX_ROWS rows is cut to a fixed, seeded sample of its rows, whose row numbers
+    are written beside it as ``<name>_rows.npy``, so two builds run with the same arguments dump the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.ndim and a.shape[0] > DUMP_MAX_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_MAX_ROWS, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.atleast_1d(a))
+
+
 def run_headline(args, rank, world, local_rank):
     import torch
 
@@ -355,6 +375,7 @@ def run_headline(args, rank, world, local_rank):
             pt = xh[j].numpy() if hasattr(xh, "numpy") else xh[j]
             return allgather_best(best_v.value, offset + j, pt)
 
+        step.values = vals_host  # the M acquisition values the last step wrote to the host
         return step
 
     # ---- clocks during the timed region ----
@@ -368,7 +389,8 @@ def run_headline(args, rank, world, local_rank):
     tg_ms, tg_n, tg_fl = C.c_double(), C.c_int64(), C.c_double()
     lib.tb_gp_profile_read(h, C.byref(tg_ms), C.byref(tg_n), C.byref(tg_fl))
     lib.tb_gp_profile(h, 0)
-    ms_e2e, _, _ = timer(step_host_fused(xc_pinned), args.steps)
+    step_pinned = step_host_fused(xc_pinned)
+    ms_e2e, _, _ = timer(step_pinned, args.steps)
     ms_e2e_pageable, _, _ = timer(step_host_fused(xc_pageable), max(1, min(args.steps, 3)))
     n_pageable = max(1, min(args.steps, 3))
 
@@ -376,6 +398,10 @@ def run_headline(args, rank, world, local_rank):
         stop_evt.set()
         th.join(timeout=10)
     clocks = summarise_clocks(clk.get("lines"))
+    if args.dump_outputs and rank == 0:
+        # device-resident path: what sharded_argmax_local returns; pinned host path: the values tb_acq_argmax wrote
+        dump_outputs(args.dump_outputs, {"best_point": res[0], "best_value": res[1], "best_index": res[2],
+                                         "ei_values": step_pinned.values.numpy()})
 
     value = total * args.steps / (ms_dev * 1e-3)
     e2e_value = total * args.steps / (ms_e2e * 1e-3)
@@ -586,6 +612,9 @@ def run_config(args, rank, world, local_rank):
     if rank == 0:
         stop_evt.set()
         th.join(timeout=10)
+        if args.dump_outputs:
+            names = ("best_value", "best_index", "best_point") if cfg == "c3" else ("best_point", "best_value", "best_index")
+            dump_outputs(args.dump_outputs, {n: a for n, a in zip(names, res) if a is not None})
         # C5 runs host-side bookkeeping between device rounds: its step time is taken from the stream events like the others;
         # the wall clock of the timed loop (incl. warm-up) is reported beside it
         line = {"metric": name, "value": units * args.steps / (ms * 1e-3), "unit": unit, "n_gpus": world, "steps": args.steps,
@@ -612,7 +641,15 @@ def main():
     ap.add_argument("--engine", default="int8", choices=["int8", "int8x21", "fp64"],
                     help="variance GEMM engine: int8 = fp64-accurate digit split on the INT8 tensor cores, product count picked from the "
                          "error estimate (default); int8x21 = the full 21 products; fp64 = native DMMA")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64; rank 0's "
+                         "values for several GPUs); headline: the winner of the device-resident path and the acquisition "
+                         "values of the pinned host path")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))

@@ -1,20 +1,19 @@
 """Extract the structural protocols of the reference's model / acquisition boundary into a JSON fixture.
 
-    python tests/golden/make_protocols.py      (needs /root/reference; writes tests/golden/reference_protocols.json)
+    python tests/golden/make_protocols.py TRIESTE_CHECKOUT/trieste      (writes tests/golden/reference_protocols.json)
 
 The reference's boundary for this path is a set of Python structural protocols (SURVEY.md §8b):
 trieste/models/interfaces.py:38-327 (ProbabilisticModel and its Supports*/Has* refinements) and
 trieste/acquisition/interface.py:27-157 (AcquisitionFunctionBuilder & co).  TensorFlow is not installable here, so the
 files are parsed with ``ast`` (never imported): for every class the fixture records its bases and, per method, the argument
 names in order (without ``self``), which of them are keyword-only and which have defaults.  tests/test_protocol_conformance.py
-checks the native classes against the fixture (and, when /root/reference is present, the fixture against the reference).
+checks the native classes against the fixture.
 """
 import ast
 import json
 import os
 import sys
 
-REF = "/root/reference/trieste"
 FILES = {
     "models/interfaces.py": ["ProbabilisticModel", "TrainableProbabilisticModel", "SupportsPredictJoint", "SupportsPredictY",
                              "SupportsGetKernel", "SupportsGetObservationNoise", "SupportsGetInternalData",
@@ -60,7 +59,7 @@ def extract(path, wanted):
     return out
 
 
-def build(ref=REF):
+def build(ref):
     fixture = {}
     for rel, wanted in FILES.items():
         fixture[rel] = extract(os.path.join(ref, rel), wanted)
@@ -68,7 +67,9 @@ def build(ref=REF):
 
 
 if __name__ == "__main__":
-    fx = build()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    fx = build(sys.argv[1])
     dst = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_protocols.json")
     json.dump(fx, open(dst, "w"), indent=1, sort_keys=True)
     print("wrote", dst, {k: sorted(v) for k, v in fx.items()}, file=sys.stderr)

@@ -1,10 +1,9 @@
 """Drop-in boundary check (CPU): every method of the reference's structural protocols for this path exists on the native
 classes with the same argument names in the same order.
 
-The protocols are read from tests/golden/reference_protocols.json, extracted with ``ast`` from
-/root/reference/trieste/models/interfaces.py:38-327, models/gpflow/interface.py and acquisition/interface.py:27-157 by
-tests/golden/make_protocols.py (the reference cannot be imported: TensorFlow is not installable).  When /root/reference is
-present the fixture itself is re-derived and compared, so it cannot go stale silently."""
+The protocols are read from tests/golden/reference_protocols.json, extracted with ``ast`` from the reference's
+trieste/models/interfaces.py:38-327, models/gpflow/interface.py and acquisition/interface.py:27-157 by
+tests/golden/make_protocols.py, so neither the reference nor TensorFlow has to be installed to run it."""
 import inspect
 import json
 import os
@@ -87,17 +86,6 @@ def test_native_class_offers_the_reference_protocol_method(cls, protocol, mname,
         assert next(p for p in positional if p.name == name).default is not inspect.Parameter.empty, (cls.__name__, mname, name)
     for name in m["kwonly"]:
         assert name in {p.name for p in params}, f"{cls.__name__}.{mname} lacks keyword argument {name!r}"
-
-
-def test_fixture_matches_the_reference_when_it_is_present():
-    if not os.path.isdir("/root/reference/trieste"):
-        pytest.skip("/root/reference is not mounted on this box")
-    import importlib.util
-
-    spec = importlib.util.spec_from_file_location("make_protocols", os.path.join(HERE, "golden", "make_protocols.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    assert mod.build() == FIXTURE, "tests/golden/reference_protocols.json is stale: re-run tests/golden/make_protocols.py"
 
 
 def test_split_acquisition_function_follows_the_reference_rule():
